@@ -2,6 +2,7 @@
 """bench.py -- headline benchmark of the batch SGP4/SDP4 path (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload config2|config3|config4]
+                    [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over the synthetic grid (BASELINE config 2 by default: 13,478
 near-earth satellites x 1,440 epochs, fp64, velocities on, TEME).  One JSON line is printed by rank 0.
@@ -24,6 +25,10 @@ near-earth satellites x 1,440 epochs, fp64, velocities on, TEME).  One JSON line
   config3 / config4   sub-records for the other BASELINE grids (mixed SGP4/SDP4 at N = 1; the week-long grid
                sharded + gathered at N > 1).
   --impl reference  times only that CPU path and prints the same line shape with "impl": "reference".
+  --dump-outputs DIR  after the timed steps, writes the position and velocity blocks of the last timed step as
+               DIR/pos.npy and DIR/vel.npy (float64, satellite-major TEME, km and km/s): the rows dump_rows() picks, a
+               fixed seeded sample when the whole block would not fit DUMP_BYTES.  The workloads are seeded, so two
+               builds (or the two --impl arms) can be compared cell for cell.  One process only (--gpus 1).
 """
 from __future__ import annotations
 
@@ -47,6 +52,22 @@ FLOP_PER_SDP4_CELL = {0: 1000.0, 1: 1500.0, 2: 1500.0}
 BYTES_PER_CELL = 48.2          # 48 B written (pos+vel) + ~0.2 B of element reads
 PUBLISHED_CPU_HEADLINE = 303e6  # props/s, astroz 16 threads on Ryzen 7 7840U (README.md:39)
 METRIC = "propagations/sec (sat x time pairs)"
+DUMP_BYTES = 48_000_000        # pos + vel written by --dump-outputs, float64: well under 64 MB
+
+
+def dump_rows(n_sats: int, n_times: int) -> np.ndarray:
+    """Satellite rows --dump-outputs writes: all of them when pos + vel fit DUMP_BYTES, else a sorted sample drawn
+    with seed 0 (config2: 694 of the 13,478 rows, every epoch)."""
+    k = min(n_sats, max(1, DUMP_BYTES // (2 * n_times * 3 * 8)))
+    if k == n_sats:
+        return np.arange(n_sats)
+    return np.sort(np.random.default_rng(0).choice(n_sats, k, replace=False))
+
+
+def write_outputs(out_dir: str, pos: np.ndarray, vel: np.ndarray) -> None:
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in (("pos", pos), ("vel", vel)):
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, dtype=np.float64))
 
 
 def _peaks():
@@ -153,7 +174,8 @@ def usable_cpus() -> dict:
 
 def cpu_reference_pass(tles, jd, fr, min_seconds: float, min_reps: int, max_reps: int, sdp4_threads: int = 0):
     """Time the CPU SIMD port (restatement of src/Sgp4Batch.zig + src/Sdp4Batch.zig + src/Constellation.zig threading)
-    on all host threads, outputs pre-touched so page faults are not billed to either arm."""
+    on all host threads, outputs pre-touched so page faults are not billed to either arm.  Also returns the time-major
+    (pos, vel) block of the last pass."""
     from oracle import oracle as orc
 
     orc.build()
@@ -169,7 +191,7 @@ def cpu_reference_pass(tles, jd, fr, min_seconds: float, min_reps: int, max_reps
         t0 = time.perf_counter()
         sim.propagate(jd, fr, layout=1, threads=threads, out=(pos, vel), sdp4_threads=sdp4_threads)
         times.append(time.perf_counter() - t0)
-    return times, threads, orc.simd_isa(), sim.numSdp4
+    return times, threads, orc.simd_isa(), sim.numSdp4, (pos, vel)
 
 
 def cpu_baseline_record(tles, jd, fr, seconds: float, min_reps: int, max_reps: int) -> dict:
@@ -177,7 +199,7 @@ def cpu_baseline_record(tles, jd, fr, seconds: float, min_reps: int, max_reps: i
     the SDP4 phase -- the reference's own (the phase gets the threads the SGP4 phase left over, i.e. one,
     src/Constellation.zig:358-364) and an even split -- and the FASTER one is the baseline."""
     cells = len(tles) * len(jd)
-    times, threads, isa, nd = cpu_reference_pass(tles, jd, fr, seconds, min_reps, max_reps, 0)
+    times, threads, isa, nd, _ = cpu_reference_pass(tles, jd, fr, seconds, min_reps, max_reps, 0)
     rec = {"value": cells * len(times) / sum(times), "unit": "props/s", "cores": threads, "kind": "port", "isa": isa,
            "host": usable_cpus(),
            "sample": f"full grid ({cells} cells) x {len(times)} passes over ~{sum(times):.0f} s, sustained mean, "
@@ -185,7 +207,7 @@ def cpu_baseline_record(tles, jd, fr, seconds: float, min_reps: int, max_reps: i
            "best_pass_value": cells / min(times),
            "published_reference": "303 M props/s (16 thr) / 37.7 M (1 thr) on Ryzen 7 7840U, README.md:39 (near-earth only)"}
     if nd:
-        t2, _, _, _ = cpu_reference_pass(tles, jd, fr, seconds, min_reps, max_reps, max(1, threads // 2))
+        t2, _, _, _, _ = cpu_reference_pass(tles, jd, fr, seconds, min_reps, max_reps, max(1, threads // 2))
         even = cells * len(t2) / sum(t2)
         rec["sdp4_thread_policy"] = {"reference_rule_value": rec["value"], "even_split_value": even,
                                      "note": "src/Constellation.zig:358-364 gives the deep-space phase only the threads "
@@ -202,12 +224,15 @@ def run_reference(args, rank: int, world: int) -> None:
     tles, jd, fr, desc = workload(args.workload)
     cells = len(tles) * len(jd)
     reps = args.warmup + args.steps
-    times, threads, isa, nd = cpu_reference_pass(tles, jd, fr, 0.0, reps, reps, 0)
+    times, threads, isa, nd, (pos, vel) = cpu_reference_pass(tles, jd, fr, 0.0, reps, reps, 0)
     policy = "reference rule"
     if nd:   # mixed catalog: also the even split of threads for the deep-space phase; keep the faster
-        t2, _, _, _ = cpu_reference_pass(tles, jd, fr, 0.0, reps, reps, max(1, threads // 2))
+        t2, _, _, _, _ = cpu_reference_pass(tles, jd, fr, 0.0, reps, reps, max(1, threads // 2))
         if sum(t2[args.warmup:]) < sum(times[args.warmup:]):
             times, policy = t2, "even split of threads between the SGP4 and SDP4 phases"
+    if args.dump_outputs:   # threads split satellites, so both policies give the same numbers; block is (nt, n, 3)
+        rows = dump_rows(len(tles), len(jd))
+        write_outputs(args.dump_outputs, pos[:, rows].transpose(1, 0, 2), vel[:, rows].transpose(1, 0, 2))
     timed = times[args.warmup:]
     total = float(sum(timed))
     value = cells * len(timed) / total
@@ -414,6 +439,10 @@ def run_ours(args, rank: int, local_rank: int, world: int) -> None:
     # ---- timed region: exactly K steps, CUDA events on the launching stream, max over ranks ----------------------
     ms_per_step = h.time_steps(step, args.steps)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs:   # the block of the last timed step, before any later leg writes it again
+        rows_d = torch.as_tensor(dump_rows(n, nt), device=dev)
+        write_outputs(args.dump_outputs, pos.index_select(0, rows_d).cpu().numpy(),
+                      vel.index_select(0, rows_d).cpu().numpy())
     if clocks is not None:
         clocks["soak_steps_before_timed_region"] = soak_steps
     value = cells / (ms_per_step * 1e-3)
@@ -750,11 +779,15 @@ def main() -> None:
     ap.add_argument("--workload", default="config2")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-subrecords", action="store_true", help="skip the config3 sub-record of the default N=1 run")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write pos.npy / vel.npy of the last timed step (sampled rows, see dump_rows) to DIR")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3)
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
+    if args.dump_outputs and world > 1:
+        raise SystemExit("--dump-outputs writes one process's result block: run it with --gpus 1")
     if args.impl == "reference":
         run_reference(args, rank, world)
     else:
